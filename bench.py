@@ -2,6 +2,7 @@
 """bench.py -- MTTKRP nnz*R/sec per mode on synthetic sparse tensors (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one MTTKRP sweep: one MTTKRP per mode of the tensor (the hot path of
 one CPD-ALS iteration).  value = nnz_total * R * nmodes / step time = the mean
@@ -37,7 +38,11 @@ Also in the JSON line:
                    (SPLATT_B200_NGPUS=N), run by rank 0 while the other ranks idle.
 
 `--impl reference` times the reference's own OpenMP mttkrp_csf (oracle/_ref,
-compiled unmodified from /root/reference) on the host cores on the same workload.
+compiled unmodified from the reference's sources) on the host cores on the same workload.
+
+`--dump-outputs DIR` writes what the headline workload's timed path computed in its
+last step, the summed output of every mode, as DIR/mttkrp_mode<m>.npy (float64,
+10000 x 32 each).  Inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -512,8 +517,9 @@ class Workload:
         torch.cuda.synchronize()
         return [c.cpu().numpy() for c in cap]
 
-    def timed(self, flush, steps, warmup):
-        """W warm-up steps, then K steps back to back; returns per-step ms, per-mode ms lists."""
+    def timed(self, flush, steps, warmup, capture=None):
+        """W warm-up steps, then K steps back to back; returns per-step ms, per-mode ms lists.
+        capture: a list of N slots that receives the outputs of the last step."""
         import torch
         for _ in range(warmup):
             flush.zero_()
@@ -529,9 +535,14 @@ class Workload:
         for k in range(steps):
             flush.zero_()
             ev[k][0].record()
-            self.sweep(kev[k])
+            # the fused exchange re-zeroes its buffer after every mode, so its result is copied
+            # inside the last step; the other paths' outputs are still in place after the loop
+            self.sweep(kev[k], capture if k == steps - 1 and self.fx is not None else None)
             ev[k][1].record()
         self.ctx.barrier()
+        if capture is not None and self.fx is None:
+            for m in range(self.N):
+                capture[m] = self.outs[m].clone()
         wall = time.time() - w0
         self.launches = S.launch_count() - l0
         step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -602,7 +613,7 @@ def run_named(ctx, key, args, flush):
     del ind, vals
     torch.cuda.empty_cache()
     ours = wl.outputs_host()
-    steps = max(5, min(args.steps, 10))
+    steps = args.steps
     step_ms, mode_ms, _ = wl.timed(flush, steps, max(args.warmup, 3))
     ms_per_step = ctx.max_over_ranks(float(np.sum(step_ms))) / steps
     per_mode = [ctx.max_over_ranks(float(np.mean(mode_ms[m]))) for m in range(wl.N)]
@@ -698,7 +709,13 @@ def run_ours(args):
     ind, vals = make_coo_gpu(nnz_total, dev)
     wl = Workload(ctx, dims, ind, vals, RANK, args.nccl_exchange, SEED)
     ours_host = wl.outputs_host()          # also warms the GPU up before the W warm-up steps
-    step_ms, kern_ms, wall_s = wl.timed(flush, args.steps, max(args.warmup, 3))
+    last = [None] * NMODES if args.dump_outputs else None
+    step_ms, kern_ms, wall_s = wl.timed(flush, args.steps, max(args.warmup, 3), capture=last)
+    if last is not None and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for m, out in enumerate(last):
+            np.save(os.path.join(args.dump_outputs, f"mttkrp_mode{m}.npy"), out.cpu().numpy())
+    del last
     launches = wl.launches
     ms_per_step = ctx.max_over_ranks(float(np.sum(step_ms))) / args.steps
     worst_step = ctx.max_over_ranks(float(np.max(step_ms)))
@@ -902,8 +919,10 @@ def run_ours(args):
         sys.stderr.flush()
         print(json.dumps(line), flush=True)
         # the JSON line must be the LAST line on stdout: with NCCL_DEBUG=INFO the library
-        # prints from its exit handlers ("Closing env plugin ...") -- leave without running them
-        os._exit(0)
+        # prints from its exit handlers ("Closing env plugin ...") -- whatever is printed from
+        # here on goes to stderr, and the process still ends through the normal interpreter
+        # exit (atexit handlers, library destructors)
+        os.dup2(sys.stderr.fileno(), sys.stdout.fileno())
     return 0
 
 
@@ -913,6 +932,9 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's per-mode outputs of the headline workload "
+                         "as DIR/mttkrp_mode<m>.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--nccl-exchange", action="store_true",
                     help="N>1: use kernel + NCCL all-reduce instead of the fused multicast exchange")

@@ -77,6 +77,10 @@ gcc -fopenmp -o "$OUT/splatt" "${cmdobjs[@]}" "${objs[@]}" \
 # splatt_mttkrp_free_ws and splatt_mttkrp from libsplatt_b200.so (INTEGRATION.md,
 # option A).  `splatt_gpu cpd ...` = reference host code + B200 MTTKRP.
 B200LIB="$HERE/../splatt_b200/libsplatt_b200.so"
+# linked by name, not path: the library has no soname, so a path on the link line would be
+# recorded as the dependency and the binaries would break once the tree moves; the
+# $ORIGIN-relative rpath below finds it in whatever directory the tree lands in
+B200LINK=(-L"$HERE/../splatt_b200" -l:libsplatt_b200.so)
 if [ -f "$B200LIB" ]; then
   objcopy --redefine-sym splatt_mttkrp_csf=splatt_mttkrp_csf_cpu \
           --redefine-sym splatt_mttkrp=splatt_mttkrp_cpu \
@@ -87,16 +91,16 @@ if [ -f "$B200LIB" ]; then
   for o in "${objs[@]}"; do
     case "$o" in */mttkrp.o) gpuobjs+=("$OUT/obj/mttkrp_cpu.o");; *) gpuobjs+=("$o");; esac
   done
-  gcc -fopenmp -o "$OUT/splatt_gpu" "${cmdobjs[@]}" "${gpuobjs[@]}" "$B200LIB" \
+  gcc -fopenmp -o "$OUT/splatt_gpu" "${cmdobjs[@]}" "${gpuobjs[@]}" "${B200LINK[@]}" \
       "$BLASLIB" -Wl,--disable-new-dtags,-rpath,"$BLASDIR" -Wl,-rpath,'$ORIGIN/../../splatt_b200' -lm -lrt
 fi
 # The reference's OWN MTTKRP unit tests (tests/mttkrp_test.c: every fixture x every mode x
 # ONEMODE/TWOMODE/ALLMODE x NOTILE/DENSETILE levels, gold = mttkrp_stream, abs tol 1e-10),
 # built twice: against the reference's kernels (reftest_mttkrp_cpu) and against
 # libsplatt_b200.so through the same symbol rename (reftest_mttkrp_gpu).  The fixture
-# directory is a fixed scratch path that tests/test_reference_unit_tests.py fills from
-# tests/golden/*.npz before running the binaries.
-FIX='"/tmp/splatt_b200_fixtures/"'
+# directory is relative to the working directory: tests/test_reference_unit_tests.py writes
+# it from tests/golden/*.npz into a temporary directory and runs the binaries there.
+FIX='"splatt_b200_fixtures/"'
 tobjs=()
 for f in main.c mttkrp_test.c; do
   o="$OUT/obj/t_${f%.c}.o"
@@ -107,7 +111,7 @@ done
 gcc -fopenmp -o "$OUT/reftest_mttkrp_cpu" "${tobjs[@]}" "${objs[@]}" \
     "$BLASLIB" -Wl,--disable-new-dtags,-rpath,"$BLASDIR" -lm -lrt
 if [ -f "$B200LIB" ]; then
-  gcc -fopenmp -o "$OUT/reftest_mttkrp_gpu" "${tobjs[@]}" "${gpuobjs[@]}" "$B200LIB" \
+  gcc -fopenmp -o "$OUT/reftest_mttkrp_gpu" "${tobjs[@]}" "${gpuobjs[@]}" "${B200LINK[@]}" \
       "$BLASLIB" -Wl,--disable-new-dtags,-rpath,"$BLASDIR" -Wl,-rpath,'$ORIGIN/../../splatt_b200' -lm -lrt
 fi
 rm -rf "$OUT/obj"

@@ -21,9 +21,7 @@ def lib():
 
 @pytest.fixture(scope="session")
 def refmod():
-    """The compiled, unmodified reference (oracle/_ref).  Skips when it was not built."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    ref.load()
-    return ref
+    """The reference's answers: the compiled, unmodified reference (oracle/_ref) where it was
+    built, otherwise its stored answers to the same calls (tests/refgold.py)."""
+    from tests import refgold
+    return refgold

@@ -1,6 +1,5 @@
 """BASELINE config 1: the UNMODIFIED reference CLI on a small 3-mode .tns, rank 16, one CPU
 thread (reference plumbing, no GPU) -- proves the oracle build is a working SPLATT."""
-import os
 import re
 import subprocess
 from pathlib import Path
@@ -9,6 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import ref
+from tests.util import relocated_binary
 
 GOLD = Path(__file__).parent / "golden"
 
@@ -63,7 +63,7 @@ def test_reference_cli_linked_against_libsplatt_b200(tmp_path, name, rank, gpus)
     SPLATT_B200_NGPUS=2 on two real GPUs (gpurun --gpus 2) -- the reference's C host driving
     several GPUs through the unchanged C API (the shape of src/mpi/mpi_cpd.c:627-804)."""
     import torch
-    env = dict(os.environ)
+    gpu_cli, env = relocated_binary(GPU_CLI, tmp_path)
     if gpus == "list-0,0":
         env["SPLATT_B200_DEVICES"] = "0,0"
     elif gpus == "ngpus-2":
@@ -76,7 +76,7 @@ def test_reference_cli_linked_against_libsplatt_b200(tmp_path, name, rank, gpus)
     args = ["cpd", str(tns), "-r", str(rank), "-t", "2", "--seed", "3", "--nowrite", "-i", "6",
             "--tol", "0"]
     cpu = subprocess.run([str(ref.CLI_PATH)] + args, capture_output=True, text=True, timeout=300)
-    gpu = subprocess.run([str(GPU_CLI)] + args, capture_output=True, text=True, timeout=300, env=env)
+    gpu = subprocess.run([str(gpu_cli)] + args, capture_output=True, text=True, timeout=300, env=env)
     assert cpu.returncode == 0 and gpu.returncode == 0, gpu.stderr
     f_cpu = re.findall(r"fit = ([0-9.]+)  delta = ([-+0-9.e]+)", cpu.stdout)
     f_gpu = re.findall(r"fit = ([0-9.]+)  delta = ([-+0-9.e]+)", gpu.stdout)
@@ -106,9 +106,10 @@ def test_reference_bench_harness_on_gpu(tmp_path, name):
     shim_c.write_text("#include <time.h>\ntime_t time(time_t * t) { if (t) *t = 1234567; return 1234567; }\n")
     shim = tmp_path / "time_shim.so"
     subprocess.run(["gcc", "-shared", "-fPIC", "-o", str(shim), str(shim_c)], check=True)
-    env = dict(os.environ, LD_PRELOAD=str(shim))
+    gpu_cli, env = relocated_binary(GPU_CLI, tmp_path)
+    env["LD_PRELOAD"] = str(shim)
     outs = {}
-    for tag, exe in (("cpu", ref.CLI_PATH), ("gpu", GPU_CLI)):
+    for tag, exe in (("cpu", ref.CLI_PATH), ("gpu", gpu_cli)):
         wd = tmp_path / tag
         wd.mkdir()
         r = subprocess.run([str(exe), "bench", str(tns), "-a", "csf", "-i", "1", "-r", "8", "-t", "2",

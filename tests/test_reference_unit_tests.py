@@ -8,9 +8,10 @@ mttkrp_stream, abs tol 1e-10, 7 OpenMP threads.
                          resolve from libsplatt_b200.so (objcopy rename, INTEGRATION.md option A):
                          the reference's test-suite judging our CUDA kernels.
 
-Both binaries are built by oracle/build_ref.sh; fixtures are rewritten from tests/golden/*.npz
-into the scratch directory the binaries were compiled to read."""
-import os
+Both binaries are built by oracle/build_ref.sh to read their fixtures from
+splatt_b200_fixtures/ under the working directory; they are rewritten there from
+tests/golden/*.npz and a relocated copy of the binary (tests/util.py) runs in a temporary
+directory."""
 import re
 import subprocess
 from pathlib import Path
@@ -19,19 +20,17 @@ import numpy as np
 import pytest
 
 from oracle import ref
+from tests.util import relocated_binary
 
 GOLD = Path(__file__).parent / "golden"
-FIX = Path("/tmp/splatt_b200_fixtures")
 CPU = ref.CLI_PATH.parent / "reftest_mttkrp_cpu"
 GPU = ref.CLI_PATH.parent / "reftest_mttkrp_gpu"
 
 
-def _write_fixtures():
-    FIX.mkdir(exist_ok=True)
+def _write_fixtures(fix):
+    fix.mkdir()
     for name in ("small", "med", "small4", "med4", "med5"):
-        out = FIX / f"{name}.tns"
-        if out.exists():
-            continue
+        out = fix / f"{name}.tns"
         z = np.load(GOLD / f"{name}.npz")
         ind, vals = z["ind"], z["vals"]
         with open(out, "w") as f:
@@ -40,14 +39,16 @@ def _write_fixtures():
                 f.write(f" {float(vals[n])!r}\n")
 
 
-def _run(exe):
-    _write_fixtures()
+def _run(exe, wd):
+    _write_fixtures(wd / "splatt_b200_fixtures")
+    exe, env = relocated_binary(exe, wd)
     # the tests ask for 7 threads, but their gold (mttkrp_stream) runs before the first
     # omp_set_num_threads call; on a 128-CPU host the default-sized team stalls in libgomp --
     # pin the default team size to what the tests intend
-    env = dict(os.environ, OMP_NUM_THREADS="7")
+    env["OMP_NUM_THREADS"] = "7"
     try:
-        r = subprocess.run([str(exe), "mttkrp"], capture_output=True, text=True, timeout=150, env=env)
+        r = subprocess.run([str(exe), "mttkrp"], capture_output=True, text=True, timeout=150, env=env,
+                           cwd=wd)
     except subprocess.TimeoutExpired:
         # seen once with a default-sized (128-thread) OpenMP team: every thread asleep inside the
         # reference's CPU gold mttkrp_stream (backtrace: GOMP barrier) -- not a verdict on the kernels
@@ -58,15 +59,15 @@ def _run(exe):
 
 
 @pytest.mark.skipif(not CPU.exists(), reason="oracle/_ref/reftest_mttkrp_cpu not built")
-def test_reference_mttkrp_unit_tests_cpu():
-    (total, ok, failed, skipped), out = _run(CPU)
+def test_reference_mttkrp_unit_tests_cpu(tmp_path):
+    (total, ok, failed, skipped), out = _run(CPU, tmp_path)
     assert (total, ok, failed, skipped) == (7, 7, 0, 0), out[-1500:]
 
 
 @pytest.mark.gpu
 @pytest.mark.skipif(not GPU.exists(), reason="oracle/_ref/reftest_mttkrp_gpu not built")
-def test_reference_mttkrp_unit_tests_on_libsplatt_b200():
-    (total, ok, failed, skipped), out = _run(GPU)
+def test_reference_mttkrp_unit_tests_on_libsplatt_b200(tmp_path):
+    (total, ok, failed, skipped), out = _run(GPU, tmp_path)
     assert (total, ok, failed, skipped) == (7, 7, 0, 0), out[-1500:]
     for name in ("csf_one_notile", "csf_two_notile", "csf_all_notile", "csf_one_densetile_alldepth",
                  "csf_two_densetile_alldepth", "csf_all_densetile_alldepth"):

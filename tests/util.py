@@ -1,7 +1,13 @@
 """Shared helpers for the test-suite: seeded synthetic tensors and error norms."""
 from __future__ import annotations
 
+import os
+import re
+from pathlib import Path
+
 import numpy as np
+
+ROOT = Path(__file__).resolve().parent.parent
 
 
 def random_coo(dims, nnz, seed=0, unique=True, skew=None):
@@ -57,3 +63,26 @@ def factor_mats(dims, R, seed=0):
 def rel_fro(a, b):
     den = np.linalg.norm(b)
     return float(np.linalg.norm(a - b) / (den if den > 0 else 1.0))
+
+
+def relocated_binary(exe, wd):
+    """A copy in `wd` of a binary under oracle/_ref that runs wherever the tree now lies, and
+    the environment to run it in.
+
+    Binaries linked by an earlier oracle/build_ref.sh name libsplatt_b200.so by the absolute
+    path of the tree they were built in, and read their fixtures from /tmp/splatt_b200_fixtures/.
+    In the copy both strings are rewritten in place (same length, NUL-padded): the library by
+    file name, found through LD_LIBRARY_PATH, and the fixtures relative to the working
+    directory.  Binaries of the current recipe already use both forms and are copied unchanged."""
+    data = Path(exe).read_bytes()
+
+    def pad(m, new):
+        return new + b"\0" * (len(m.group(0)) - len(new))
+    data = re.sub(rb"/[^\0]*/splatt_b200/libsplatt_b200\.so\0",
+                  lambda m: pad(m, b"libsplatt_b200.so\0"), data)
+    data = re.sub(rb"/tmp/(splatt_b200_fixtures/[^\0]*\0)", lambda m: pad(m, m.group(1)), data)
+    out = Path(wd) / Path(exe).name
+    out.write_bytes(data)
+    out.chmod(0o755)
+    paths = [str(ROOT / "splatt_b200")] + [p for p in [os.environ.get("LD_LIBRARY_PATH")] if p]
+    return out, dict(os.environ, LD_LIBRARY_PATH=os.pathsep.join(paths))
